@@ -6,8 +6,11 @@ every step's frames are exchanged inside the timed region and the clip is comple
 Prints ONE JSON line on rank 0; DESIGN.md §5 explains every field.  The same line carries, under roofline.extra.configs, short measurements
 of BASELINE configs[1] (render only) and configs[4] (48+48 samples + the torso/background SR head) so that one driver run records them.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
+
+--dump-outputs DIR writes the frames the last timed step returned to DIR/frames.npy, so that two builds run with the same arguments (and
+therefore the same seeded inputs) can be compared output for output.
 """
 import argparse
 import hashlib
@@ -18,6 +21,7 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -29,6 +33,19 @@ RENDER_BYTES_PER_FRAME = 26.51e6     # fused render, S=48: planes 25.17 MB + jit
 RENDER_GFLOP_PER_FRAME = 1.84        # decoder 1.636 GFLOP + ~0.2 GFLOP interpolation / composite (SURVEY.md §8d)
 WARP_CONV_GFLOP_PER_FRAME = 782.0    # torso head conv stack without the torso warper (SURVEY.md §8d); 685 with the per-clip cache
 METRIC = 'rendered frames/sec @512^2 (64^2 NeRF, 48 samples/ray)'
+DUMP_BYTES = 64 * 10 ** 6            # --dump-outputs budget: larger outputs keep a seeded selection of whole frames
+
+
+def dump_frames(out_dir, frames):
+    """frames [F,...] (fp32 or uint8) -> out_dir/frames.npy in float32.  Above DUMP_BYTES a fixed seeded selection of whole frames is kept
+    (in frame order), the same selection for every run with the same arguments."""
+    a = frames.detach().float().cpu()
+    per_frame = a[0].numel() * a.element_size()
+    if a.numel() * a.element_size() > DUMP_BYTES:
+        keep = torch.randperm(a.shape[0], generator=torch.Generator().manual_seed(0))[:max(1, DUMP_BYTES // per_frame)]
+        a = a[keep.sort().values]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, 'frames.npy'), a.numpy())
 
 
 def peaks():
@@ -289,7 +306,13 @@ def main():
     ap.add_argument('--no-extra-configs', action='store_true', help='skip the configs[1] / configs[4] mini-benchmarks')
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-graph', action='store_true', help='launch every kernel from Python instead of replaying one CUDA graph per step')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='after the timed steps, write the frames of the last timed step to DIR/frames.npy '
+                                                          '(float32; above 64 MB a seeded selection of whole frames)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs writes the frames of the GPU path; it does not apply to --impl reference')
     args.warmup = max(args.warmup, 3)
     if args.impl == 'reference':
         return run_reference(args)
@@ -353,8 +376,11 @@ def main():
             exchange_note += 'fell back to the NCCL all-gather'
     eng.prepare(resident)                                                    # one step graph per resident batch: inputs are read in place
 
+    last = [None]                                                            # what the last step returned (the engine reuses the buffer)
+
     def step(i):
-        return eng.step(*resident[i % nb], frame_index=((i - args.warmup) % args.steps) * B if i >= args.warmup else 0)
+        last[0] = eng.step(*resident[i % nb], frame_index=((i - args.warmup) % args.steps) * B if i >= args.warmup else 0)
+        return last[0]
 
     sampler = ClockSampler(local); sampler.start()
     launches0 = L.r3dp_launch_count()
@@ -362,6 +388,8 @@ def main():
     launches = L.r3dp_launch_count() - launches0
     if eng.graph is not None or eng.inplace:        # kernels replayed from the captured graph are not re-counted by the library
         launches = eng.launches_per_step * args.steps
+    if args.dump_outputs and rank == 0:
+        dump_frames(args.dump_outputs, last[0])
     if exchange == 'p2p':
         eng.close_clip()
     fps = world * B * args.steps / (ms / 1e3)

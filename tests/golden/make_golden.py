@@ -236,6 +236,20 @@ def large_sr_case():
     save('sr_large', image=img, seeds=np.array([8]), n_res=2)
 
 
+def ref_small_case():
+    """The reference's renderer wired as oracle/ref_runner.py runs it for the CPU baseline: N=1, 3x32x32x32 planes, 16^2 rays, 12 (+12)
+    samples; inputs come from seeds."""
+    N, res, S = 1, 16, 12
+    planes, cam = syn.make_planes(N, h=32, w=32, seed=0), syn.make_cameras(N, seed=1)
+    dec = ref_decoder(syn.make_decoder_params(seed=4))
+    out = {}
+    for S_imp in (0, 12):
+        u_c, u_f = syn.make_jitter(N, res * res, S, S_imp, seed=2)
+        _, _, rgb, depth, wsum, valid = ref_render(planes, dec, cam, res, S, S_imp, u_c, u_f)
+        out.update({f'imp{S_imp}.rgb': rgb, f'imp{S_imp}.depth': depth, f'imp{S_imp}.wsum': wsum, f'imp{S_imp}.valid': valid})
+    save('render_ref_small', res=res, S=S, seeds=np.array([0, 1, 2, 4]), **out)
+
+
 def load(name):
     return np.load(os.path.join(HERE, name + '.npz'))
 
@@ -252,6 +266,9 @@ if __name__ == '__main__':
     if len(sys.argv) > 1 and sys.argv[1] == 'trigrid':
         trigrid_case()
         sys.exit(0)
+    if len(sys.argv) > 1 and sys.argv[1] == 'ref_small':
+        ref_small_case()
+        sys.exit(0)
     small_cases()
     layer_cases()
     full_cases()
@@ -259,3 +276,4 @@ if __name__ == '__main__':
     warp_case('v1'); warp_case('v3')
     trigrid_case()
     large_sr_case()
+    ref_small_case()
