@@ -245,7 +245,9 @@ int r3dp_sr_tc_last_layer_ex(const void* x_f16, const void* wp_f16, const float*
  * The reference SR computes in fp32 (networks_stylegan2.py:37-94, conv2d_resample.py:48-145).  These entry points keep that accuracy on
  * tcgen05: every fp32 operand is stored as two fp16 halves v = hi + lo (activations NHWC [N,H,W, 2*Cpad] = [hi | lo]; packed weights
  * [Nw,taps,O, 2*Ipad] = [hi | lo] of w * 2^10) and every convolution accumulates hi*hi + lo*hi + hi*lo in fp32 (three times the MMAs; the
- * dropped lo*lo term is ~2^-22).  Same arguments and meaning as the r3dp_sr_tc_* functions of the same name; tensors are twice as wide. */
+ * dropped lo*lo term is ~2^-22).  Same arguments and meaning as the r3dp_sr_tc_* functions of the same name; tensors are twice as wide.
+ * Activations are split unscaled, so results are fp32-grade (within 2x of an fp32 evaluation) for layer inputs of magnitude 2^-4 and above;
+ * below that the lo halves become fp16 subnormals and the error grows (~1.7e-5 of max|y| at 2^-10, tests/test_cpu_split_conv.py). */
 int r3dp_sr_tcx_pack_weights(const float* wf, int Nw, int O, int I, void* packed_f16, r3dp_stream_t stream);
 int r3dp_sr_tcx_pack_weights_up_composed(const float* wf, int Nw, int O, int I, void* packed_f16, r3dp_stream_t stream);
 int r3dp_sr_tcx_input(const float* x, int N, int C, int h, int w, int size, void* y_f16, r3dp_stream_t stream);

@@ -1085,7 +1085,7 @@ static int run_conv2(const void* x, int N, int H, int W, int Cp, const void* wp,
     a.k_chunks = Cp / BK; a.tiles_x = W / BM; a.n_blocks = O / BN; a.n_images = N; a.w_shared = (Nw == 1);
     { static int mixv = -1; if (mixv < 0) { const char* e = getenv("R3DP_TC_MIX"); mixv = (e && e[0] == '0') ? 0 : 1; } a.phase_mix = mixv; }      // A/B knob
     if (a.act_gain == 0.f) { a.act_slope = 0.2f; a.act_gain = 1.4142135623730951f; }      // default: bias_act lrelu
-    R3DP_REQUIRE(a.n_blocks >= 1 && a.n_blocks <= 2, "conv_tc3: 128 or 256 output channels");
+    R3DP_REQUIRE(a.n_blocks >= 1 && a.n_blocks <= 2, "conv_tc3: needs Cout == 128 or Cout == 256 (got Cout=%d)", O);
     return tc_rows() == 1 ? launch_conv3_r<1>(tmA, tmB, a, max_rows, st) : (tc_rows() == 4 ? launch_conv3_r<4>(tmA, tmB, a, max_rows, st) : launch_conv3_r<2>(tmA, tmB, a, max_rows, st));
 }
 
@@ -1158,9 +1158,10 @@ extern "C" size_t r3dp_sr_tcx_scratch_bytes(int N, int O, int H, int W) { return
 static int layer_impl(const void* x_f16, const void* wp_f16, const float* bias, int N, int Nw, int I, int O, int H, int W, int up,
                       void* y_f16, void* scratch, int split, r3dp_stream_t stream) {
     R3DP_REQUIRE(x_f16 && wp_f16 && bias && y_f16, "sr_tc_layer: null pointer");
-    R3DP_REQUIRE(N > 0 && (Nw == N || Nw == 1) && I > 0 && H > 0, "sr_tc_layer: bad shape");
+    R3DP_REQUIRE(N > 0 && (Nw == N || Nw == 1) && I > 0 && H > 0, "sr_tc_layer: bad shape (needs N, I, H > 0 and Nw == N or Nw == 1; got N=%d, Nw=%d, I=%d, H=%d)",
+                 N, Nw, I, H);
     R3DP_REQUIRE(W % BM == 0 && O % BN == 0, "sr_tc_layer: needs W %% 128 == 0 and Cout %% 128 == 0 (got W=%d, Cout=%d)", W, O);
-    R3DP_REQUIRE(up == 1 || up == 2, "sr_tc_layer: up must be 1 or 2");
+    R3DP_REQUIRE(up == 1 || up == 2, "sr_tc_layer: up must be 1 or 2 (got up=%d)", up);
     const int Ip = (I + 63) / 64 * 64;
     cudaStream_t st = as_stream(stream);
     ConvArgs a = {};
@@ -1172,11 +1173,16 @@ static int layer_impl(const void* x_f16, const void* wp_f16, const float* bias, 
         a.out = reinterpret_cast<__half*>(y_f16); a.out_H = H; a.out_W = W; a.out_C = O; a.oy_mul = a.ox_mul = 1;
         return launch_conv(x_f16, N, H, W, Ip, wp_f16, Nw, O, a, st);
     }
+    // every check of the up=2 path runs before its first launch: a rejected call enqueues nothing and leaves the scratch untouched
     R3DP_REQUIRE(scratch, "sr_tc_layer: up=2 needs scratch");
+    R3DP_REQUIRE(Ip <= 256, "sr_tc_layer: up=2 supports at most 256 input channels");
+    R3DP_REQUIRE((2 * W) % FIR_TW == 0 && O % 64 == 0, "sr_tc_layer: FIR needs 2W %% 32 == 0 and Cout %% 64 == 0");
     __half* yb = reinterpret_cast<__half*>(scratch);
+    CUtensorMap tmY, tmY8;
+    if (make_map_fir(&tmY, yb, (uint64_t)O * (split ? 2 : 1), (uint64_t)(2 * W + 1), (uint64_t)(2 * H + 1), (uint64_t)N, FIR_BH)) return 1;
+    if (make_map_fir(&tmY8, yb, (uint64_t)O * (split ? 2 : 1), (uint64_t)(2 * W + 1), (uint64_t)(2 * H + 1), (uint64_t)N, FIR_TH)) return 1;
     if (launch_upconv2(x_f16, N, H, W, Ip, wp_f16, Nw, O, yb, bias, split, st)) return 1;
     {
-        R3DP_REQUIRE(Ip <= 256, "sr_tc_layer: up=2 supports at most 256 input channels");
         const int erows = split ? kEdgeRowsSplit : kEdgeRows;
         dim3 grid((2 * H + 1 + erows - 1) / erows, (O + kEdgeCo - 1) / kEdgeCo, N);
         const size_t esmem = ((size_t)(kEdgeRows / 2 + 2) * Ip + 3 * (size_t)kEdgeCo * (Ip + 8)) * sizeof(__half);
@@ -1192,10 +1198,6 @@ static int layer_impl(const void* x_f16, const void* wp_f16, const float* bias, 
         }
     }
     {
-        R3DP_REQUIRE((2 * W) % FIR_TW == 0 && O % 64 == 0, "sr_tc_layer: FIR needs 2W %% 32 == 0 and Cout %% 64 == 0");
-        CUtensorMap tmY, tmY8;
-        if (make_map_fir(&tmY, yb, (uint64_t)O * (split ? 2 : 1), (uint64_t)(2 * W + 1), (uint64_t)(2 * H + 1), (uint64_t)N, FIR_BH)) return 1;
-        if (make_map_fir(&tmY8, yb, (uint64_t)O * (split ? 2 : 1), (uint64_t)(2 * W + 1), (uint64_t)(2 * H + 1), (uint64_t)N, FIR_TH)) return 1;
         const int total = N * (O / 64) * ((2 * H + FIR_SEG - 1) / FIR_SEG) * (2 * W / FIR_TW);
         if (split) {
             const int smem = 4 * FIR_SLOT + 1024 + 64;
@@ -1227,7 +1229,8 @@ static int last_layer_impl(const void* x_f16, const void* wp_f16, const float* b
                            const float* img_prev, int N, int Nw, int I, int H, int W, float* img_out, uint8_t* img_out_u8, int clamp, int split,
                            r3dp_stream_t stream) {
     R3DP_REQUIRE(x_f16 && wp_f16 && bias && wrgb && brgb && (img_out || img_out_u8), "sr_tc_last_layer: null pointer");
-    R3DP_REQUIRE(N > 0 && (Nw == N || Nw == 1) && W % BM == 0 && H % 2 == 0, "sr_tc_last_layer: bad shape");
+    R3DP_REQUIRE(N > 0 && (Nw == N || Nw == 1) && W % BM == 0 && H % 2 == 0,
+                 "sr_tc_last_layer: bad shape (needs N > 0, Nw == N or Nw == 1, W %% 128 == 0, H %% 2 == 0; got N=%d, Nw=%d, H=%d, W=%d)", N, Nw, H, W);
     const int Ip = (I + 63) / 64 * 64;
     ConvArgs a = {};
     a.bias = bias; a.wrgb = wrgb; a.brgb = brgb; a.img_prev = img_prev; a.img_out = img_out; a.img_out_u8 = img_out_u8; a.out_clamp = clamp || img_out_u8;
@@ -1275,7 +1278,9 @@ static int layer_torgb_impl(const void* x_f16, const void* wp_f16, const float* 
                             const float* img_prev, int N, int Nw, int I, int O, int H, int W, void* y_f16, float* img_out, int split,
                             r3dp_stream_t stream) {
     R3DP_REQUIRE(x_f16 && wp_f16 && bias && wrgb && brgb && y_f16 && img_out, "sr_tc_layer_torgb: null pointer");
-    R3DP_REQUIRE(N > 0 && (Nw == N || Nw == 1) && W % BM == 0 && O % BN == 0 && O <= 256 && H % 2 == 0, "sr_tc_layer_torgb: bad shape");
+    R3DP_REQUIRE(N > 0 && (Nw == N || Nw == 1) && W % BM == 0 && O % BN == 0 && O <= 256 && H % 2 == 0,
+                 "sr_tc_layer_torgb: bad shape (needs N > 0, Nw == N or Nw == 1, W %% 128 == 0, Cout 128 or 256, H %% 2 == 0; got N=%d, Nw=%d, Cout=%d, H=%d, W=%d)",
+                 N, Nw, O, H, W);
     const int Ip = (I + 63) / 64 * 64;
     Conv2Args a = {};
     Taps t = {};
@@ -1416,7 +1421,8 @@ extern "C" int r3dp_sr_tcx_pack_weights_up_composed(const float* wf, int Nw, int
 static int layer_up_composed_impl(const void* x_f16, const void* wpc_f16, const float* bias, int N, int Nw, int I, int O, int H,
                                   int W, void* y_f16, int split, r3dp_stream_t stream) {
     R3DP_REQUIRE(x_f16 && wpc_f16 && bias && y_f16, "sr_tc_layer_up_composed: null pointer");
-    R3DP_REQUIRE(N > 0 && (Nw == N || Nw == 1) && W % BM == 0 && O % BN == 0 && O <= 256, "sr_tc_layer_up_composed: bad shape");
+    R3DP_REQUIRE(N > 0 && (Nw == N || Nw == 1) && W % BM == 0 && O % BN == 0 && O <= 256,
+                 "sr_tc_layer_up_composed: bad shape (needs N > 0, Nw == N or Nw == 1, W %% 128 == 0, Cout 128 or 256; got N=%d, Nw=%d, Cout=%d, W=%d)", N, Nw, O, W);
     const int Ip = (I + 63) / 64 * 64;
     Conv2Args a = {};
     a.n_phases = 4;
@@ -1447,8 +1453,10 @@ extern "C" int r3dp_sr_tcx_layer_up_composed(const void* x_f16, const void* wpc_
 static int conv_res_impl(const void* x_f16, const void* wp_f16, const float* bias, int N, int Nw, int I, int O, int H, int W, int ksize,
                          int act, const void* residual_f16, void* y_f16, int split, r3dp_stream_t stream) {
     R3DP_REQUIRE(x_f16 && wp_f16 && bias && y_f16, "sr_tc_conv: null pointer");
-    R3DP_REQUIRE(N > 0 && (Nw == N || Nw == 1) && W % BM == 0 && O % BN == 0 && O <= 256 && (ksize == 1 || ksize == 3) && act >= 0 && act <= 3,
-                 "sr_tc_conv: bad shape / options");
+    R3DP_REQUIRE(N > 0 && (Nw == N || Nw == 1) && W % BM == 0 && O % BN == 0 && O <= 256,
+                 "sr_tc_conv: bad shape (needs N > 0, Nw == N or Nw == 1, W %% 128 == 0, Cout 128 or 256; got N=%d, Nw=%d, Cout=%d, W=%d)", N, Nw, O, W);
+    R3DP_REQUIRE(ksize == 1 || ksize == 3, "sr_tc_conv: ksize must be 1 or 3 (got %d)", ksize);
+    R3DP_REQUIRE(act >= 0 && act <= 3, "sr_tc_conv: act must be 0..3 (got %d)", act);
     const int Ip = (I + 63) / 64 * 64;
     Conv2Args a = {};
     Taps t = {};
@@ -1484,7 +1492,8 @@ extern "C" int r3dp_sr_tc_layer_torgb_noup(const void* x_f16, const void* wp_f16
                                            const float* img_prev, int N, int Nw, int I, int O, int H, int W, void* y_f16, float* img_out,
                                            r3dp_stream_t stream) {
     R3DP_REQUIRE(x_f16 && wp_f16 && bias && wrgb && brgb && y_f16 && img_out, "sr_tc_layer_torgb_noup: null pointer");
-    R3DP_REQUIRE(N > 0 && (Nw == N || Nw == 1) && W % BM == 0 && O % BN == 0 && O <= 256, "sr_tc_layer_torgb_noup: bad shape");
+    R3DP_REQUIRE(N > 0 && (Nw == N || Nw == 1) && W % BM == 0 && O % BN == 0 && O <= 256,
+                 "sr_tc_layer_torgb_noup: bad shape (needs N > 0, Nw == N or Nw == 1, W %% 128 == 0, Cout 128 or 256; got N=%d, Nw=%d, Cout=%d, W=%d)", N, Nw, O, W);
     const int Ip = (I + 63) / 64 * 64;
     Conv2Args a = {};
     Taps t = {};
@@ -1643,7 +1652,8 @@ __global__ void alpha_gate_kernel(const __half* __restrict__ y, int stride, int 
     out[pix] = fminf(sg, cap[pix]);
 }
 extern "C" int r3dp_sr_alpha_gate(const void* logits_f16, int stride, int lo_off, const float* cap, int N, int H, int W, float* out, r3dp_stream_t stream) {
-    R3DP_REQUIRE(logits_f16 && cap && out && N > 0 && H > 0 && W > 0 && stride > 0 && lo_off >= 0 && lo_off < stride, "sr_alpha_gate: bad arguments");
+    R3DP_REQUIRE(logits_f16 && cap && out && N > 0 && H > 0 && W > 0, "sr_alpha_gate: bad arguments");
+    R3DP_REQUIRE(stride > 0 && lo_off >= 0 && lo_off < stride, "sr_alpha_gate: needs 0 <= lo_off < stride (got lo_off=%d, stride=%d)", lo_off, stride);
     const long long npix = (long long)N * H * W;
     alpha_gate_kernel<<<(unsigned)((npix + 255) / 256), 256, 0, as_stream(stream)>>>(reinterpret_cast<const __half*>(logits_f16), stride, lo_off, cap, npix, out);
     R3DP_LAUNCH_CHECK();

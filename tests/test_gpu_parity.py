@@ -207,7 +207,10 @@ def _tc_layer_case(up, I, O, H, W, N=2, shared=False, seed=0, composed=False):
 
 
 @pytest.mark.parametrize('up,I,O,H,W,shared', [(1, 64, 128, 6, 128, False), (1, 256, 256, 5, 256, True), (2, 32, 128, 5, 128, False),
-                                               (2, 256, 128, 4, 256, False)])
+                                               (2, 256, 128, 4, 256, False),
+                                               # odd row-group count (padded to even), I not a multiple of 64, two cout blocks, two-step up at H=5
+                                               (1, 64, 128, 5, 128, False), (1, 96, 128, 4, 128, True), (1, 64, 256, 4, 128, False),
+                                               (2, 128, 128, 5, 128, True)])
 def test_tc_layer_vs_oracle(up, I, O, H, W, shared):
     got, ref = _tc_layer_case(up, I, O, H, W, shared=shared)
     assert got.shape == ref.shape
@@ -243,13 +246,28 @@ def test_sr_tc_per_sample_styles_vs_fp32_path():
     assert err < 5e-3 * rng, (err, rng)
 
 
-def test_sr_full_tc_exact_vs_reference(golden):
+def test_sr_full_tc_exact_vs_reference(golden, monkeypatch):
     """sr_mode='tc_exact': the same tensor-core kernels with split fp16 operands (hi*hi + lo*hi + hi*lo, fp32 accumulation) must reproduce the
-    reference's fp32 image to fp32 grade: stated bar 1e-3 * range (the judge's bar for an 'exact' tensor-core mode); measured ~1e-5."""
+    reference's fp32 image to fp32 grade: stated bar 1e-3 * range (the judge's bar for an 'exact' tensor-core mode); measured ~1e-5.
+    Also prints max|x| of every conv layer's input: the split activations are unscaled, so the path is fp32-grade only while they stay at
+    2^-4 and above (include/r3dp_b200.h, tests/test_cpu_split_conv.py)."""
+    from real3dportrait_b200 import sr_tc
+    seen, layer = [], sr_tc.layer
+
+    def spy(x16, lay, wp, up, split=False):            # inputs and outputs of the two up layers = the inputs of all four conv layers
+        y = layer(x16, lay, wp, up, split)
+        for t in (x16, y):
+            c = t.shape[-1] // 2
+            seen.append(float((t[..., :c].float() + t[..., c:].float()).abs().max()))
+        return y
+    monkeypatch.setattr(sr_tc, 'layer', spy)
     fimg = orc.feature_image(golden('render_full48')['rgb'], 64).to(DEV)
     sr = r3.SuperresolutionHybrid8XDC(channels=32, img_resolution=512, sr_num_fp16_res=0, sr_antialias=True, sr_mode='tc_exact')
     sr.load_state_dict(syn.make_sr_params(seed=5), strict=True)
     img = sr.to(DEV)(fimg[:, :3], fimg, torch.ones(1, 14, 512, device=DEV), noise_mode='none')
+    assert len(seen) == 4
+    print('tc_exact SR layer inputs max|x|: ' + ', '.join(f'{n} {v:.3g}' for n, v in zip(('block0.conv0', 'block0.conv1', 'block1.conv0',
+                                                                                           'block1.conv1'), seen)))
     ref = golden('sr_full')['image']
     err, rng = _maxdiff(img, ref), float(ref.max() - ref.min())
     print(f'tc_exact SR: max-abs {err:.3e} on range {rng:.2f}')
